@@ -5,7 +5,7 @@ A "step" = one pass of the hot path over one 512x512-ray x 64-sample frame per G
 rays -> sample points -> skinning-voxel sample -> inverse LBS -> PE -> 9-layer SDF MLP -> per-ray first
 hit.  Inputs are seeded synthetic data of the BASELINE shapes (no dataset / checkpoint exists offline).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--mode tc3|tc1|simt] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--mode tc3|tc1|simt] [--impl reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.
 """
@@ -31,6 +31,7 @@ MODES = {"simt": 0, "tc3": 1, "tc1": 2}
 # ncu capture of the final round-1 kernel, profiles/r01_ncu_tc3_current.txt (142.3 MB read + 54.8 MB written; the
 # algorithmic minimum is the 67 MB sdf output + the touched part of the 181 MB voxel + 8.6 MB of weights)
 TRAFFIC_BYTES = {"tc3": 197053696}
+DUMP_SDF_RAYS = 65536   # rays of the per-sample SDF written by --dump-outputs (all 512x512 of them would be 64 MiB)
 
 
 def measured_peaks():
@@ -338,6 +339,19 @@ def secondary_rates(dev, ren, mode):
     }
 
 
+def dump_outputs(out_dir, sdf, hit_idx, hit_t):
+    """What render() returned in the last timed step, as <out_dir>/<name>.npy: the per-ray first-hit sample index
+    (float64, exact) and distance of every ray, and the per-sample SDF of a fixed seeded sample of DUMP_SDF_RAYS rays
+    (ascending ray order).  The inputs are seeded, so two builds run with the same arguments can be compared file by file."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    R = sdf.shape[0]
+    rows = torch.randperm(R, generator=torch.Generator().manual_seed(0))[:DUMP_SDF_RAYS].sort().values
+    arrays = {"sdf": sdf[rows.to(sdf.device)].float(), "hit_idx": hit_idx.double(), "hit_t": hit_t.float()}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
+
+
 _JSON_OUT = None
 
 
@@ -372,7 +386,13 @@ def main():
     ap.add_argument("--frames", type=int, default=1, help="frames per step of the strong-scaling job (4 = configs[3])")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write the last step's render outputs to DIR/<name>.npy (rank 0's rays)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; the reference arm has none")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -470,6 +490,8 @@ def main():
     launches = ops.launch_count() - launches0
     ops.check_async_errors()
     sampler.stop_flag = True
+    if args.dump_outputs and rank == 0:   # before the e2e leg: render() reuses its sdf buffer
+        dump_outputs(args.dump_outputs, sdf, hit_idx, hit_t)
     step_ms = [a.elapsed_time(b) for a, b in ev]
     dev_s = max_over_ranks(t_beg.elapsed_time(t_end) * 1e-3)   # device time of the K steps, max over ranks
     ms_per_step = dev_s * 1e3 / args.steps

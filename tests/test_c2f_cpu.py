@@ -1,14 +1,12 @@
-"""CPU: the re-implemented coarse-to-fine sweep returns the reference's grid bit-for-bit when both use
-the same query function (reference class imported through oracle/refload.py -- container only), and
-the committed golden grid pins it on machines without /root/reference."""
+"""CPU: the re-implemented coarse-to-fine sweep returns the reference's grid and lattice geometry bit-for-bit when
+both use the same query function (tests/golden/c2f_grid.npz and c2f_lattice.npz hold what the reference class
+computes, tests/golden/make_golden_c2f.py)."""
 import os
 
 import numpy as np
-import pytest
 import torch
 
-from conftest import GOLDEN
-from oracle import refload
+from conftest import GOLDEN, load_golden
 from recmv_b200.MCAcc import Seg3dLossless, create_grid3D
 
 
@@ -45,15 +43,13 @@ def test_matches_golden_grid():
     assert sum(s[3] for s in eng.stats) < 0.4 * 49 * 97 * 65  # and it evaluates a fraction of the lattice
 
 
-@pytest.mark.skipif(not refload.available(), reason="needs /root/reference (container only)")
 def test_bit_identical_to_reference_class():
-    ns = refload.load()
-    ref = ns.MCAcc.Seg3dLossless(sphere_query, **KW)
+    grid, lattice = load_golden("c2f_grid.npz")["grid"], load_golden("c2f_lattice.npz")
     ours = Seg3dLossless(sphere_query, **KW)
-    a, b = ref.forward(), ours.forward()
-    assert torch.equal(a, b)
+    b = ours.forward()
+    assert torch.equal(b, torch.from_numpy(grid)[None, None])
     for name in ("spacing_x", "spacing_y", "spacing_z", "bx", "by", "bz"):
-        assert getattr(ref, name) == getattr(ours, name)
+        assert float(lattice[name]) == getattr(ours, name)
 
 
 def test_interp2x_boundary_oracle_pins():
