@@ -327,6 +327,21 @@ RECMV_API int recmv_fragment_decode(const int64_t* pix_to_face, const float* bar
                           int64_t* out_col, float* out_pts, int64_t* out_finds, float* out_rays, int32_t* counters,
                           recmv_stream_t stream);
 
+/* ---- mesh rasteriser: what `maskRender` gets from pytorch3d's MeshRasterizer (model/network.py:307-322; faces_per_pixel=1,
+ * blur_radius=0, perspective_correct=True, no culling), in the camera convention of model/CameraMine.py:146-173 --------------
+ * verts [N,V,3] f32 (N posed meshes sharing faces [F,3] int64), cam = host float[4] {fx, fy, px, py} shared by all frames,
+ * R [NR,3,3] row-major and T [NR,3] device f32 with NR = 1 or N: Xc = Xw R + T, screen x = px - fx Xc/Zc, y = py - fy Yc/Zc,
+ * pixel (row, col) = screen point (x = col, y = row).  A face covers a pixel when its three screen-space barycentrics at the
+ * pixel centre are > 0 (either winding) and its three vertices have Zc > 0; zero-area faces cover nothing.  Winner: smallest
+ * perspective-correct Zc, then smallest face index (deterministic).  Outputs (pytorch3d layout, -1 on background):
+ * pix_to_face [N,H,W] int64 = n*F + f, zbuf [N,H,W] f32 = Zc, bary [N,H,W,3] f32 perspective-correct, vertex order of
+ * the face.  Faces with a clipped bounding box over 128 pixels are swept by a warp.  Face indices must be in range.
+ * scratch: recmv_raster_scratch_bytes(N, H, W) bytes.  Two kernels + one memset, no host synchronisation.           */
+RECMV_API int recmv_raster_scratch_bytes(int N, int H, int W, size_t* bytes /*host*/);
+RECMV_API int recmv_rasterize(const float* verts, const int64_t* faces, int N, int64_t V, int64_t F,
+                    const float* cam /*host float[4]: fx fy px py*/, const float* R, const float* T, int NR, int H, int W,
+                    void* scratch, int64_t* pix_to_face, float* zbuf, float* bary, recmv_stream_t stream);
+
 /* ---- A11 / (f2): the sweep of one pyramid level as a DEVICE WORKLIST (SURVEY 8b `recmv_c2f_sweep`) -----------------
  * replaces the coordinate-list bookkeeping of MCAcc/seg3d_lossless.py:306-428 (nonzero / unique / index scatter, a
  * host sync per step).  level / final_res are (W, H, D) = (x, y, z) lattice sizes (host).

@@ -2,6 +2,7 @@
 raise on non-zero status, wire autograd.  PyTorch is plumbing here (device memory, streams,
 autograd graph); all arithmetic happens in librecmv_b200.so.
 """
+import collections
 import ctypes
 from ctypes import byref, c_float, c_int64, c_size_t
 
@@ -1254,6 +1255,48 @@ def fragment_decode(pix_to_face, bary, verts, faces, mask=None, camera=None):
     n = int(counters.item())
     out = (ob[:n], orow[:n], ocol[:n], opts[:n], ofi[:n])
     return out + (orays[:n],) if camera is not None else out
+
+
+Fragments = collections.namedtuple("Fragments", ["pix_to_face", "zbuf", "bary_coords", "dists"])
+
+
+def rasterize(verts, faces, camera, image_size):
+    """Mesh rasteriser (recmv_rasterize): one face per pixel, the convention of pytorch3d's MeshRasterizer with
+    faces_per_pixel=1, blur_radius=0, perspective_correct=True and no culling, in the reference camera's pixel grid
+    (CameraMine.project / view_rays: pixel (row, col) is the screen point (col, row)).
+    verts [N,V,3] (or [V,3]: one mesh) float32, faces [F,3] int64 shared by the N meshes, both CUDA and contiguous;
+    camera = (fx, fy, px, py, R [NR,3,3] or [3,3], T [NR,3] or [3]) with NR = 1 or N; image_size = (H, W) or an int.
+    Returns Fragments(pix_to_face [N,H,W,1] int64 packed n*F + f, zbuf [N,H,W,1] camera-space Zc, bary_coords
+    [N,H,W,1,3] perspective-correct, dists=None), -1 everywhere on background."""
+    _check_input(verts, "verts")
+    _check_input(faces, "faces")
+    if verts.dtype != torch.float32 or faces.dtype != torch.int64:
+        raise RuntimeError("rasterize: verts must be float32 and faces int64")
+    if verts.dim() == 2:
+        verts = verts.unsqueeze(0)
+    if verts.dim() != 3 or verts.shape[2] != 3 or faces.dim() != 2 or faces.shape[1] != 3:
+        raise RuntimeError("rasterize: expected verts [N,V,3] or [V,3] and faces [F,3]")
+    H, W = (image_size, image_size) if isinstance(image_size, int) else (int(image_size[0]), int(image_size[1]))
+    N, V = verts.shape[0], verts.shape[1]
+    fx, fy, px, py, R, T = camera
+    dev = verts.device
+    R = torch.as_tensor(R, dtype=torch.float32, device=dev).reshape(-1, 3, 3).contiguous()
+    T = torch.as_tensor(T, dtype=torch.float32, device=dev).reshape(-1, 3).contiguous()
+    if R.shape[0] != T.shape[0]:
+        raise RuntimeError("rasterize: R and T must hold the same number of cameras")
+    lib = _lib.load()
+    nbytes = c_size_t(0)
+    check(lib.recmv_raster_scratch_bytes(N, H, W, byref(nbytes)), "recmv_raster_scratch_bytes")
+    scratch = torch.empty((nbytes.value,), dtype=torch.uint8, device=dev)
+    p2f = torch.empty((N, H, W, 1), dtype=torch.int64, device=dev)
+    zbuf = torch.empty((N, H, W, 1), dtype=torch.float32, device=dev)
+    bary = torch.empty((N, H, W, 1, 3), dtype=torch.float32, device=dev)
+    cam = (c_float * 4)(float(fx), float(fy), float(px), float(py))
+    with torch.cuda.device(dev):
+        check(lib.recmv_rasterize(_ptr(verts), _ptr(faces), N, V, int(faces.shape[0]), cam, _ptr(R), _ptr(T),
+                                  int(R.shape[0]), H, W, _ptr(scratch), _ptr(p2f), _ptr(zbuf), _ptr(bary), _stream(verts)),
+              "recmv_rasterize")
+    return Fragments(p2f, zbuf, bary, None)
 
 
 class C2fLevel:

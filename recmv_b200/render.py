@@ -10,6 +10,9 @@ voxel, skeleton) and exposes
 Sharding (`shard_rows`): rays are independent given replicated weights / voxel / bone matrices
 (SURVEY 8e), so ranks take contiguous blocks of image rows (or whole frames) and there is NO
 data-path collective; gradients -- when training -- are exchanged by `allreduce_grads`.
+
+`MaskRasterizer` / `render_colors`: from a (marching-cubes) mesh to rasteriser fragments and to the colour frame of
+`infer_garment`, on the device (`ops.rasterize`, csrc/raster.cu).
 """
 import torch
 
@@ -184,3 +187,67 @@ class SdfRenderer:
                              {"renderRatio": ratio.get("renderRatio") if isinstance(ratio, dict) else ratio})
         rgb.index_copy_(0, idx, col)
         return rgb, hit, t
+
+
+# ---- mesh rasterisation and the colour frame of infer_garment ---------------------------------------------------------
+class MaskRasterizer:
+    """The `maskRender` of the reference (model/network.py:307-322) for the call sites that read only the fragments,
+    `__, frags = self.maskRender(meshes)` (OptimGarmentNetwork.py:767,1397,1448,1492; OptimNetwork.py:437): callable on
+    (verts [N,V,3] | [V,3], faces [F,3]) or on a meshes object with verts_padded() / faces_padded() whose faces are the
+    same for every mesh.  Returns (None, ops.Fragments) -- no shaded image.
+    camera = (fx, fy, px, py, R, T) as for ops.rasterize; image_size = (H, W)."""
+
+    def __init__(self, camera, image_size):
+        self.camera = camera
+        self.image_size = image_size
+
+    def __call__(self, meshes, faces=None):
+        if faces is None:
+            verts, fp = meshes.verts_padded(), meshes.faces_padded()
+            faces = fp[0]
+            if not all(torch.equal(f, faces) for f in fp[1:]):
+                raise RuntimeError("MaskRasterizer: every mesh must have the same face list")
+        else:
+            verts = meshes
+        return None, ops.rasterize(verts.detach().contiguous(), faces.contiguous(), self.camera, self.image_size)
+
+
+def render_colors(canon_verts, faces, sdf_net, deformer, defconds, render_net, camera, image_size, ratio, ang_threshold,
+                  offset_type=None, dthreshold=1e-4, times=30, chunk=10000):
+    """The colour branch of infer_garment (OptimGarmentNetwork.py:3128-3204) on the device: deform the canonical mesh
+    for the N frames of `defconds`, rasterise, seed points + view rays (FindSurfacePsRays), surface solve per chunk of
+    `chunk` rays, canonical normal from the fused value+gradient launch, cardinal rays, colour network, and
+    clamp((c/2 + 0.5) * 255) scattered into a white [N,H,W,3] image.  The rays and the camera position use camera 0
+    (cam_pos = -R[0] T[0]), as the reference does.  Returns (colors [N,H,W,3] float, mask [N,H,W] bool, fragments)."""
+    from . import utils
+    fx, fy, px, py, R, T = camera
+    R = torch.as_tensor(R, dtype=torch.float32, device=canon_verts.device).reshape(-1, 3, 3)
+    T = torch.as_tensor(T, dtype=torch.float32, device=canon_verts.device).reshape(-1, 3)
+    N = defconds[1][0].shape[0]
+    H, W = (image_size, image_size) if isinstance(image_size, int) else image_size
+    with torch.no_grad():
+        verts = canon_verts.detach().contiguous()
+        def_verts = deformer(verts[None].expand(N, -1, 3), defconds, ratio=ratio, offset_type=offset_type)
+        frags = ops.rasterize(def_verts.contiguous(), faces, (fx, fy, px, py, R, T), (H, W))
+        b, r, c, seeds, _, rays = utils.FindSurfacePsRays(verts, faces, frags, (fx, fy, px, py, R[0].cpu()))
+        cam_pos = -R[0].matmul(T[0].view(3, 1)).view(3)
+    cols = []
+    for rays_, seeds_, b_ in zip(torch.split(rays, chunk), torch.split(seeds, chunk), torch.split(b, chunk)):
+        if rays_.shape[0] == 0:
+            continue
+        ps, _ = utils.OptimizeGarmentSurfaceSinlge(cam_pos, rays_, seeds_.clone(), b_, sdf_net, ratio, deformer, defconds,
+                                                   dthreshold=dthreshold, athreshold=ang_threshold, w1=3.05, w2=1.,
+                                                   times=times, offset_type=offset_type)
+        with torch.no_grad():
+            _, g = sdf_net.value_and_grad(ps, ratio, want_feat=True)
+            feat = sdf_net.rendcond
+            nx = g / g.norm(dim=1, keepdim=True)
+        crays, _ = utils.compute_cardinal_rays(deformer, ps, rays_, defconds, b_, ratio, 'test', offset_type=offset_type)
+        with torch.no_grad():
+            cols.append(render_net(ps, nx, crays, feat, ratio))
+    with torch.no_grad():
+        tcolors = torch.cat(cols, 0) if cols else torch.zeros((0, 3), device=canon_verts.device)
+        tcolors = torch.clamp((tcolors / 2. + 0.5) * 255., min=0., max=255.)
+        colors = torch.full((N, H, W, 3), 255., device=canon_verts.device)
+        colors[b, r, c, :] = tcolors
+    return colors, frags.pix_to_face[..., 0] >= 0, frags
