@@ -118,6 +118,16 @@ SIGNATURES = {
     "recmv_raster_scratch_bytes": (c_int, [c_int, c_int, c_int, POINTER(c_size_t)]),
     "recmv_rasterize": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int64, POINTER(c_float), c_void_p, c_void_p, c_int,
                                 c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "recmv_points_scratch_bytes": (c_int, [c_int, c_int64, c_int, c_int, POINTER(c_size_t)]),
+    "recmv_points_count": (c_int, [c_void_p, c_int, c_int64, POINTER(c_float), c_void_p, c_void_p, c_int, c_int, c_int,
+                                   c_float, c_void_p, POINTER(c_int64), c_void_p]),
+    "recmv_points_render": (c_int, [c_void_p, c_int, c_int, c_int64, c_int, c_int, c_float, c_int, c_void_p, c_void_p,
+                                    c_int64, c_void_p, c_void_p]),
+    "recmv_points_render_backward": (c_int, [c_void_p, c_int, c_int64, POINTER(c_float), c_void_p, c_void_p, c_int, c_int,
+                                             c_int, c_float, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p,
+                                             c_void_p, c_void_p]),
+    "recmv_points_fragments": (c_int, [c_int, c_int64, c_int, c_int, c_float, c_int, c_void_p, c_void_p, c_void_p,
+                                       c_void_p, c_void_p, c_void_p]),
     "recmv_c2f_done_up": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
     "recmv_c2f_compact": (c_int, [c_void_p, POINTER(c_int), POINTER(c_int), POINTER(c_float), POINTER(c_float), c_void_p,
                                   c_void_p, c_void_p, c_int, c_void_p]),

@@ -5,7 +5,7 @@ namespace recmv {
 unsigned long long g_launch_count = 0;
 }
 
-extern "C" int recmv_version(void) { return 101; }  // 0.1.1: + recmv_rasterize
+extern "C" int recmv_version(void) { return 102; }  // 0.1.2: + recmv_points_*
 
 extern "C" int64_t recmv_launch_count(void) { return (int64_t)recmv::g_launch_count; }
 

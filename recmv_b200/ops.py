@@ -1299,6 +1299,122 @@ def rasterize(verts, faces, camera, image_size):
     return Fragments(p2f, zbuf, bary, None)
 
 
+def _camera_tensors(camera, dev):
+    fx, fy, px, py, R, T = camera
+    R = torch.as_tensor(R, dtype=torch.float32, device=dev).detach().reshape(-1, 3, 3).contiguous()
+    T = torch.as_tensor(T, dtype=torch.float32, device=dev).detach().reshape(-1, 3).contiguous()
+    if R.shape[0] != T.shape[0]:
+        raise RuntimeError("R and T must hold the same number of cameras")
+    return (c_float * 4)(float(fx), float(fy), float(px), float(py)), R, T
+
+
+class PointFragments:
+    """The selection of one `rasterize_points` call.  The dense pytorch3d layout -- idx [N,H,W,K] int64 (packed n*P + p),
+    zbuf [N,H,W,K] (camera-space Zc) and dists [N,H,W,K] (squared NDC distance), -1 in empty slots, nearest first -- is
+    expanded on the device on first access (recmv_points_fragments): at 4 x 1080^2 with K = 50 it takes 3.7 GB.
+    `candidates` is the number of (point, pixel) coverings before the per-pixel selection."""
+
+    def __init__(self, meta, scratch, cand, candidates):
+        self._meta, self._scratch, self._cand = meta, scratch, cand
+        self.candidates = candidates
+        self._dense = None
+
+    def _expand(self):
+        if self._dense is None:
+            N, P, H, W, radius, K = self._meta
+            dev = self._scratch.device
+            idx = torch.empty((N, H, W, K), dtype=torch.int64, device=dev)
+            zbuf = torch.empty((N, H, W, K), dtype=torch.float32, device=dev)
+            dists = torch.empty((N, H, W, K), dtype=torch.float32, device=dev)
+            with torch.cuda.device(dev):
+                check(_lib.load().recmv_points_fragments(N, P, H, W, radius, K, _ptr(self._scratch), _ptr(self._cand),
+                                                         _ptr(idx), _ptr(zbuf), _ptr(dists), _stream(idx)),
+                      "recmv_points_fragments")
+            self._dense = (idx, zbuf, dists)
+        return self._dense
+
+    @property
+    def idx(self):
+        return self._expand()[0]
+
+    @property
+    def zbuf(self):
+        return self._expand()[1]
+
+    @property
+    def dists(self):
+        return self._expand()[2]
+
+
+class _RasterizePointsFunction(torch.autograd.Function):
+    """images = composite(points); differentiable in `points` only (features and camera are constants)."""
+
+    @staticmethod
+    def forward(ctx, points, features, cam, R, T, size, radius, K, out):
+        N, P = points.shape[0], points.shape[1]
+        H, W = size
+        C = features.shape[1]
+        dev = points.device
+        lib = _lib.load()
+        nbytes = c_size_t(0)
+        check(lib.recmv_points_scratch_bytes(N, P, H, W, byref(nbytes)), "recmv_points_scratch_bytes")
+        scratch = torch.empty((nbytes.value,), dtype=torch.uint8, device=dev)
+        total = c_int64(0)
+        images = torch.empty((N, H, W, C), dtype=torch.float32, device=dev)
+        with torch.cuda.device(dev):
+            st = _stream(points)
+            check(lib.recmv_points_count(_ptr(points), N, P, cam, _ptr(R), _ptr(T), int(R.shape[0]), H, W, radius,
+                                         _ptr(scratch), byref(total), st), "recmv_points_count")
+            cand = torch.empty((max(total.value, 1),), dtype=torch.int64, device=dev)
+            check(lib.recmv_points_render(_ptr(features), C, N, P, H, W, radius, K, _ptr(scratch), _ptr(cand),
+                                          total.value, _ptr(images), st), "recmv_points_render")
+        ctx.save_for_backward(points, features, R, T, scratch, cand)
+        ctx.meta = (cam, size, radius, K)
+        out.append(PointFragments((N, P, H, W, radius, K), scratch, cand, total.value))
+        return images
+
+    @staticmethod
+    def backward(ctx, grad_images):
+        if not ctx.needs_input_grad[0]:
+            return (None,) * 9
+        points, features, R, T, scratch, cand = ctx.saved_tensors
+        cam, (H, W), radius, K = ctx.meta
+        N, P = points.shape[0], points.shape[1]
+        grad_images = grad_images.contiguous().float()
+        grad_points = torch.empty_like(points)
+        with torch.cuda.device(points.device):
+            check(_lib.load().recmv_points_render_backward(
+                _ptr(points), N, P, cam, _ptr(R), _ptr(T), int(R.shape[0]), H, W, radius, _ptr(features),
+                int(features.shape[1]), K, _ptr(scratch), _ptr(cand), _ptr(grad_images), _ptr(grad_points),
+                _stream(points)), "recmv_points_render_backward")
+        return (grad_points,) + (None,) * 8
+
+
+def rasterize_points(points, features, camera, image_size, radius, points_per_pixel=50):
+    """Points rasteriser + alpha compositor (recmv_points_*): pytorch3d's PointsRasterizer + AlphaCompositor
+    (background_color=None) as `pcRender` uses them, in the reference camera's pixel grid (pixel (row, col) is the screen
+    point (col, row), as ops.rasterize).  points [N,P,3] (or [P,3]: one cloud) float32 and features [P,C] float32
+    (1 <= C <= 4, the same for every cloud), both CUDA and contiguous; camera = (fx, fy, px, py, R [NR,3,3] or [3,3],
+    T [NR,3] or [3]) with NR = 1 or N, a constant; radius in NDC units (a disc of radius * min(H, W) / 2 pixels);
+    1 <= points_per_pixel <= 64.  Differentiable in `points` only: features that require grad are refused.
+    Returns (images [N,H,W,C], PointFragments).  One host synchronisation (the candidate count)."""
+    if features.requires_grad:
+        raise RuntimeError("rasterize_points: no gradient with respect to features; pass features.detach()")
+    _check_input(points, "points")
+    _check_input(features, "features")
+    if points.dtype != torch.float32 or features.dtype != torch.float32:
+        raise RuntimeError("rasterize_points: points and features must be float32")
+    if points.dim() == 2:
+        points = points.unsqueeze(0)
+    if points.dim() != 3 or points.shape[2] != 3 or features.dim() != 2 or features.shape[0] != points.shape[1]:
+        raise RuntimeError("rasterize_points: expected points [N,P,3] or [P,3] and features [P,C]")
+    size = (image_size, image_size) if isinstance(image_size, int) else (int(image_size[0]), int(image_size[1]))
+    cam, R, T = _camera_tensors(camera, points.device)
+    out = []
+    images = _RasterizePointsFunction.apply(points, features, cam, R, T, size, float(radius), int(points_per_pixel), out)
+    return images, out[0]
+
+
 class C2fLevel:
     """Device worklist of one pyramid level (recmv_c2f_refine / recmv_sdf_mlp_fwd_counted / recmv_c2f_scatter_list /
     recmv_c2f_mark_conflicts): one fused full-grid pass builds the level and its worklist, conflict rounds are driven by

@@ -13,6 +13,9 @@ data-path collective; gradients -- when training -- are exchanged by `allreduce_
 
 `MaskRasterizer` / `render_colors`: from a (marching-cubes) mesh to rasteriser fragments and to the colour frame of
 `infer_garment`, on the device (`ops.rasterize`, csrc/raster.cu).
+
+`PointsRenderer`: the point-cloud silhouette renderer `pcRender` of the training step's mask loss, on the device and
+differentiable in the point positions (`ops.rasterize_points`, csrc/points.cu).
 """
 import torch
 
@@ -251,3 +254,40 @@ def render_colors(canon_verts, faces, sdf_net, deformer, defconds, render_net, c
         colors = torch.full((N, H, W, 3), 255., device=canon_verts.device)
         colors[b, r, c, :] = tcolors
     return colors, frags.pix_to_face[..., 0] >= 0, frags
+
+
+# ---- point-cloud silhouettes of the training step's mask loss ----------------------------------------------------------
+class PointsRenderer:
+    """The reference's `pcRender` (OptimNetwork.py:87-100): PointsRendererWithFrags / PointsRendererWithFrags_Split
+    (model/CameraMine.py:306-415) over PointsRasterizer + AlphaCompositor(background_color=None).
+    camera = (fx, fy, px, py, R, T) as for ops.rasterize_points, settable between calls; image_size = (H, W) or an int;
+    radius in NDC units (`point_render.radius`).  Call on points [N,P,3], a list of N [P,3] tensors or an object with
+    points_list() (equal-size clouds), with features [P,C] (None: ones [P,1]).  Returns (images [N,H,W,C], fragments);
+    with split_size= and all_size= the `_Split` form: ([upper [N,H,W,C], lower [N,H,W,C]], fragments), upper holding the
+    points with p % all_size < split_size, both composited in one launch.  Differentiable in the points."""
+
+    def __init__(self, camera, image_size, radius, points_per_pixel=50):
+        self.camera = camera
+        self.image_size = image_size
+        self.radius = radius
+        self.points_per_pixel = points_per_pixel
+
+    def __call__(self, point_clouds, features=None, split_size=None, all_size=None):
+        if hasattr(point_clouds, "points_list"):
+            point_clouds = point_clouds.points_list()
+        points = torch.stack(list(point_clouds)) if isinstance(point_clouds, (list, tuple)) else point_clouds
+        points = points.float().contiguous()
+        P = points.shape[-2]
+        if features is None:
+            features = torch.ones((P, 1), dtype=torch.float32, device=points.device)
+        if split_size is not None:
+            if all_size is None or all_size <= 0 or P % all_size:
+                raise RuntimeError("PointsRenderer: all_size must divide the number of points of a cloud")
+            upper = (torch.arange(P, device=points.device) % all_size < split_size)[:, None]
+            features = torch.cat([features * upper, features * ~upper], 1)
+        images, frags = ops.rasterize_points(points, features.float().contiguous(), self.camera, self.image_size,
+                                             self.radius, self.points_per_pixel)
+        if split_size is not None:
+            C = images.shape[-1] // 2
+            return [images[..., :C], images[..., C:]], frags
+        return images, frags
